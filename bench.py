@@ -2,6 +2,7 @@
 """bench.py — benchmark of the path-tracing hot path (BASELINE.json metric: Mpaths/s and Mrays/s per scene).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--only]
+                    [--dump-outputs DIR]
 
 One "step" = one complete render of a workload (every sample of every pixel) through pt_render, or one pass of
 the fixed ray batch through pt_trace_batch_device.
@@ -10,8 +11,14 @@ The JSON line's HEADLINE (metric / value / ms_per_step / roofline / e2e / cpu_ba
 `10_final_720p_8192` = BASELINE configs[0] exactly: taichi_pathtracer/10_final (RTIOW random-spheres scene, 486 spheres,
 defocus blur) at the script's 1280x720, 8192 spp, depth 32.  The same line carries `workloads`: one entry per other
 BASELINE config — `8_refract_1080p` (configs[1]), `yoimiya_1080p` (configs[2]), `zhongli_4k_4096` (configs[3]),
-`intersect_10m` (configs[4]) — each with value / ms_per_step / roofline / e2e measured the same way (up to 3 timed steps).
+`intersect_10m` (configs[4]) — each with value / ms_per_step / roofline / e2e measured the same way (K timed steps).
 `--only` measures just `--workload`.
+
+--dump-outputs DIR writes what the last timed step of `--workload` computed, as the caller of that path receives it, to
+DIR/<name>.npy: `accum.npy` (a render: the [H*W, 4] float32 accumulator, RGB sums over all samples + the count of
+contributing paths) or `t.npy`, `prim.npy`, `uv.npy` (the ray batch: hit distance, primitive id as float64, barycentrics).
+Inputs are seeded, so two builds can be compared output for output.  Past 64 MB the same seeded sample of rows is written
+for every array, with the row numbers in `sample_rows.npy`.  N > 1: rank 0's arrays (for a render, the reduced image).
 
 N > 1 (torchrun, one rank per GPU): STRONG scaling for every workload — the job is fixed, the scene is replicated, the
 samples of every pixel (the rays of the batch) are split N ways, and the per-GPU accumulators are summed onto rank 0 by
@@ -59,6 +66,7 @@ KERNEL_OF = {"10_final_720p_8192": "k_paths_persist<V2>", "10_final_720p": "k_pa
 B_PER_SEGMENT = 160  # extend 48 (read o|d 32, write hit 16) + shade 112 (read o|d 32 + throughput 16 + hit 16, write successor 48)
 B_PER_PATH = 24      # fp32 RGB accumulate read-modify-write
 L2_BYTES = 126e6
+DUMP_BYTES = 63 * 10**6   # --dump-outputs: rows written in all; with the .npy headers the dump stays under 64 MB
 
 
 def measured_peaks():
@@ -273,6 +281,21 @@ class Dist:
             dist.destroy_process_group()
 
 
+def dump_outputs(directory, rows, arrays):
+    """Saves each device array of `arrays` (all with `rows` rows) as <directory>/<name>.npy; over DUMP_BYTES, the rows of
+    one seeded sample (row numbers in sample_rows.npy)."""
+    import torch
+    os.makedirs(directory, exist_ok=True)
+    per_row = sum(a.element_size() * (a.numel() // rows) for a in arrays.values())
+    if per_row * rows > DUMP_BYTES:
+        keep = np.sort(np.random.default_rng(0).choice(rows, DUMP_BYTES // (per_row + 8), replace=False))
+        np.save(os.path.join(directory, "sample_rows.npy"), keep.astype(np.float64))
+        idx = torch.from_numpy(keep).to(next(iter(arrays.values())).device)
+        arrays = {k: a[idx] for k, a in arrays.items()}
+    for k, a in arrays.items():
+        np.save(os.path.join(directory, k + ".npy"), a.cpu().numpy())
+
+
 def issue_entry(nc):
     if not nc:
         return None
@@ -283,7 +306,7 @@ def issue_entry(nc):
             "source": nc.get("summary"), "captured_from_sources": kernel_source_hash()}
 
 
-def measure_render(D, name, steps, warmup, args, cpu_seconds=0.0):
+def measure_render(D, name, steps, warmup, args, cpu_seconds=0.0, dump=None):
     """One render workload on D.world_size GPUs (strong scaling: the job's spp split over the ranks)."""
     import learn_path_tracing_b200 as L
     from learn_path_tracing_b200.multigpu import render_split_reduce, split_samples
@@ -317,6 +340,8 @@ def measure_render(D, name, steps, warmup, args, cpu_seconds=0.0):
         torch.cuda.synchronize()
         times.append(ev0.elapsed_time(ev1))
     clocks = sampler.result()
+    if dump and rank == 0:
+        dump_outputs(dump, W * H, {"accum": r.accum})
     t_local = float(sum(times))
     t_max = D.max_f(t_local)
     my_off, my_spp = split_samples(spp, ws, rank)
@@ -407,7 +432,7 @@ def measure_render(D, name, steps, warmup, args, cpu_seconds=0.0):
     return entry
 
 
-def measure_intersect(D, name, steps, warmup, args):
+def measure_intersect(D, name, steps, warmup, args, dump=None):
     """BASELINE configs[4]: fixed ray batch against an LBVH over random triangles, intersection only.  Rays and
     triangles come from counter-based device generators (bit-identical to the oracle's); N > 1 shards the batch by ray
     ranges, no collective."""
@@ -443,6 +468,8 @@ def measure_intersect(D, name, steps, warmup, args):
         torch.cuda.synchronize()
         times.append(ev0.elapsed_time(ev1))
     clocks = sampler.result()
+    if dump and rank == 0:
+        dump_outputs(dump, n_local, {"t": hits[:, 0], "prim": hits.view(torch.int32)[:, 1].double(), "uv": hits[:, 2:4]})
     t_local = float(sum(times))
     t_max = D.max_f(t_local)
     st = ctx.trace_batch_device(sc, my.data_ptr(), n_local, hits.data_ptr(), L.PT_FLAG_COUNTERS | args.trace_flags)
@@ -508,10 +535,10 @@ def measure_intersect(D, name, steps, warmup, args):
     return entry
 
 
-def measure(D, name, steps, warmup, args, cpu_seconds=0.0):
+def measure(D, name, steps, warmup, args, cpu_seconds=0.0, dump=None):
     if name in INTERSECT:
-        return measure_intersect(D, name, steps, warmup, args)
-    return measure_render(D, name, steps, warmup, args, cpu_seconds)
+        return measure_intersect(D, name, steps, warmup, args, dump)
+    return measure_render(D, name, steps, warmup, args, cpu_seconds, dump)
 
 
 def merge_clocks(a, b):
@@ -525,14 +552,15 @@ def merge_clocks(a, b):
 
 def run_ours(args):
     D = Dist()
-    head = measure(D, args.workload, args.steps, args.warmup, args, cpu_seconds=0.0 if args.no_cpu else 12.0)
+    head = measure(D, args.workload, args.steps, args.warmup, args, cpu_seconds=0.0 if args.no_cpu else 12.0,
+                   dump=args.dump_outputs)
     others = {}
     if not args.only:
         for name in OTHERS:
             if name == args.workload:
                 continue
             try:
-                others[name] = measure(D, name, min(args.steps, 3), args.warmup, args)
+                others[name] = measure(D, name, args.steps, args.warmup, args)
             except FileNotFoundError as e:  # scene caches are derived from the reference checkout (tools/prepare_assets.py)
                 others[name] = {"unavailable": str(e)}
     if D.rank == 0:
@@ -573,7 +601,11 @@ def main():
     ap.add_argument("--trace-flags", type=int, default=0, help="intersect workloads: PT_FLAG_* for pt_trace_batch_device")
     ap.add_argument("--no-cpu", action="store_true", help="skip the CPU baseline leg (profiling runs)")
     ap.add_argument("--spp", type=int, default=0, help="A/B runs only: override the workload's samples per pixel (config.spp shows it)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step of --workload computed to DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     global SPP_OVERRIDE
     SPP_OVERRIDE = max(0, args.spp)
     if args.impl == "reference":

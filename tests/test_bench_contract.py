@@ -55,14 +55,38 @@ def test_stale_ncu_counters_are_refused(tmp_path, monkeypatch):
     assert bench.ncu_counters("yoimiya_1080p")[0] == {"issue_active_pct": 70}
 
 
+import numpy as np  # noqa: E402
 import pytest  # noqa: E402
 
 
+def test_dump_outputs_writes_every_array_or_one_seeded_sample_of_rows(tmp_path, monkeypatch):
+    import torch
+    arrays = {"a": torch.arange(4000, dtype=torch.float32).reshape(1000, 4), "p": torch.arange(1000, dtype=torch.float64)}
+    bench.dump_outputs(str(tmp_path / "all"), 1000, arrays)
+    assert sorted(os.listdir(tmp_path / "all")) == ["a.npy", "p.npy"]
+    assert np.array_equal(np.load(tmp_path / "all" / "a.npy"), arrays["a"].numpy())
+    monkeypatch.setattr(bench, "DUMP_BYTES", 100 * (16 + 8 + 8))
+    for d in ("one", "two"):
+        bench.dump_outputs(str(tmp_path / d), 1000, arrays)
+    rows = np.load(tmp_path / "one" / "sample_rows.npy")
+    assert len(rows) == 100 and np.all(np.diff(rows) > 0) and np.array_equal(rows, np.load(tmp_path / "two" / "sample_rows.npy"))
+    a, p = np.load(tmp_path / "one" / "a.npy"), np.load(tmp_path / "one" / "p.npy")
+    assert a.dtype == np.float32 and p.dtype == np.float64
+    assert np.array_equal(a, arrays["a"].numpy()[rows.astype(np.int64)]) and np.array_equal(p, rows)
+    assert sum(os.path.getsize(tmp_path / "one" / f) for f in os.listdir(tmp_path / "one")) <= 100 * 32 + 3 * 128
+
+
+def test_steps_below_one_are_refused():
+    p = _run({}, "--impl", "reference", "--steps", "0")
+    assert p.returncode != 0 and "--steps" in p.stderr
+
+
 @pytest.mark.gpu
-def test_ours_arm_prints_the_contract_line_on_the_gpu():
+def test_ours_arm_prints_the_contract_line_on_the_gpu(tmp_path):
     """`bench.py --workload X --only` on the GPU: every key the driver reads is there, the roofline block carries the
-    achieved / peak / frac / traffic fields, e2e counts host<->device bytes, clocks were sampled during the timed region."""
-    p = _run({}, "--workload", "9_dof_720p", "--only", "--steps", "2", "--warmup", "3", "--no-cpu")
+    achieved / peak / frac / traffic fields, e2e counts host<->device bytes, clocks were sampled during the timed region;
+    --dump-outputs writes the accumulator of the last timed step."""
+    p = _run({}, "--workload", "9_dof_720p", "--only", "--steps", "2", "--warmup", "3", "--no-cpu", "--dump-outputs", str(tmp_path))
     assert p.returncode == 0, p.stderr[-3000:]
     line = json.loads(p.stdout.strip().splitlines()[-1])
     need = (KEYS - {"impl"}) | {"clocks", "roofline", "roofline_fp32", "mrays_per_s", "workloads", "library"}
@@ -77,3 +101,6 @@ def test_ours_arm_prints_the_contract_line_on_the_gpu():
     assert e["value"] <= 1.05 * line["value"]            # end to end cannot beat the device-resident rate
     assert line["gpu_launches"] == 2 and line["value"] > 1000 and line["clocks"]["sm_max_mhz"]
     assert line["library"]["kernel_source_hash"] == bench.kernel_source_hash()
+    acc = np.load(tmp_path / "accum.npy")
+    assert sorted(os.listdir(tmp_path)) == ["accum.npy"] and acc.dtype == np.float32 and acc.shape == (1280 * 720, 4)
+    assert np.isfinite(acc).all() and acc[:, 3].max() <= 256 and acc[:, :3].mean() > 0   # 256 spp: one whole render

@@ -1,6 +1,7 @@
 """GPU tests at BASELINE.json's FULL sizes, every config by name: configs[0] 10_final 1280x720, configs[1] 8_refract
 1080p/256 spp, configs[2] Yoimiya 1080p with the full 2048^2-per-map atlas, configs[3] Zhongli / Ganyu at 3840x2160,
-configs[4] 10 M triangles / 64 Mi rays.  The image of every render config is compared with the CPU oracle at the bench
+configs[4] 10 M triangles / 64 Mi rays (the mesh configs through the seeded stand-ins of tests/helpers.py:STAND_INS, whose
+map sizes and resolutions are the configs' own).  The image of every render config is compared with the CPU oracle at the bench
 resolution (at a sample count the oracle finishes in seconds: per-pixel 3 sigma where the count allows it, 8x8-block
 3 sigma for the 2-8 spp mesh renders); the full sample counts are covered by size-independent properties — the union
 of sample ranges equals one render, every kernel form traces the same paths, hit records are self-consistent."""
@@ -11,7 +12,7 @@ import pytest
 
 import learn_path_tracing_b200 as L
 from learn_path_tracing_b200 import scenes
-from helpers import CACHE, cached_world, hit_tolerance, mesh_camera
+from helpers import hit_tolerance, mesh_camera, stand_in_world
 
 pytestmark = pytest.mark.gpu
 
@@ -49,8 +50,7 @@ def test_config0_10_final_720p_image_within_3_sigma_of_oracle(ctx, oracle):
 
 
 def _legacy_fullsize_parity(ctx, oracle, cache, W, H, spp, max_frac):
-    world = cached_world(cache)
-    assert world is not None, f"scenes_cache/{cache}.npz missing: run tools/prepare_assets.py where the reference checkout is mounted"
+    world = stand_in_world(cache)
     cam = mesh_camera((W, H))
     r = L.Renderer(W, H, ctx, want_sq=True)
     st = r.render(world.device_scene(ctx), cam.to_struct(), spp, 32, L.PT_SHADE_LEGACY, seed=1)
@@ -73,15 +73,15 @@ def _legacy_fullsize_parity(ctx, oracle, cache, W, H, spp, max_frac):
 
 
 def test_config2_yoimiya_1080p_full_atlas_image_within_3_sigma_of_oracle(ctx, oracle):
-    """configs[2] at bench settings — 1920x1080, the full atlas (2048^2 per map), sky.png environment, depth 32 — at
-    8 of the 512 spp: the GPU LBVH + Moller-Trumbore + LUT-decoded 8-bit atlas against the oracle walking the file's own
-    SAH tree with the reference triangle test and float texels."""
+    """configs[2] at bench settings — 1920x1080, 2048^2 per map, sky environment, depth 32 — at 8 of the 512 spp, on
+    the Yoimiya stand-in: the GPU LBVH + Moller-Trumbore + LUT-decoded 8-bit atlas against the oracle walking the stored
+    tree with the reference triangle test and float texels."""
     _legacy_fullsize_parity(ctx, oracle, "yoimiya_ground_full", 1920, 1080, 8, 0.01)
 
 
 @pytest.mark.parametrize("cache", ["zhongli_full", "ganyu_full"])
 def test_config3_4k_mesh_scene_image_within_3_sigma_of_oracle(ctx, oracle, cache):
-    """configs[3] at bench resolution (3840x2160, depth 32) at 2 of the 4096 spp, both models."""
+    """configs[3] at bench resolution (3840x2160, depth 32) at 2 of the 4096 spp, the stand-ins of both models."""
     _legacy_fullsize_parity(ctx, oracle, cache, 3840, 2160, 2, 0.012)
 
 
@@ -162,7 +162,7 @@ def test_config2_yoimiya_1080p_512spp_properties(ctx):
     """configs[2] at full size: sample ranges are additive, the persistent and split kernels agree, every path
     is accounted for (the accumulator's 4th channel counts contributing paths)."""
     W, H, SPP, DEPTH = 1920, 1080, 512, 32
-    world = cached_world("yoimiya_ground_full")
+    world = stand_in_world("yoimiya_ground_full")
     cam = mesh_camera((W, H))
     sc = world.device_scene(ctx)
     full = L.Renderer(W, H, ctx)

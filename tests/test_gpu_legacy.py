@@ -4,7 +4,7 @@ import numpy as np
 import pytest
 
 import learn_path_tracing_b200 as L
-from helpers import all_triangles, cached_world, mesh_camera, synthetic_legacy_world
+from helpers import all_triangles, mesh_camera, stand_in_world, synthetic_legacy_world
 
 pytestmark = pytest.mark.gpu
 
@@ -82,9 +82,7 @@ def test_synthetic_scene_hits_match_reference_traversal(ctx, oracle):
 
 @pytest.mark.parametrize("name", ["demo", "yoimiya_ground_small", "zhongli_small", "ganyu_small"])
 def test_cached_scene_hits_match_reference_traversal(ctx, oracle, name):
-    world = cached_world(name)
-    if world is None:
-        pytest.skip("scene cache not built (tools/prepare_assets.py needs the reference checkout)")
+    world = stand_in_world(name)
     W, H = 240, 160
     cam = mesh_camera((W, H))
     if name == "demo":
@@ -130,9 +128,7 @@ def test_synthetic_scene_image_within_3_sigma(ctx, oracle, absorptivity):
 
 @pytest.mark.parametrize("name,spp", [("demo", 128), ("yoimiya_ground_small", 64), ("zhongli_small", 64), ("ganyu_small", 64)])
 def test_cached_scene_image_within_3_sigma(ctx, oracle, name, spp):
-    world = cached_world(name)
-    if world is None:
-        pytest.skip("scene cache not built")
+    world = stand_in_world(name)
     W, H = 120, 80
     cam = mesh_camera((W, H))
     if name == "demo":

@@ -7,7 +7,7 @@ import pytest
 
 import learn_path_tracing_b200 as L
 from learn_path_tracing_b200 import legacy, scene_cache, worldnpy
-from helpers import all_triangles, cached_world, synthetic_legacy_world
+from helpers import all_triangles, stand_in_world, synthetic_legacy_world
 
 REF = "/root/reference"
 needs_ref = pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout not mounted (GPU box)")
@@ -166,9 +166,7 @@ def test_lbvh_to_reference_tree_schema():
 
 def test_legacy_oracle_tree_walk_equals_brute_force(oracle):
     """The reference traversal over the stored SAH tree must find what a loop over all faces finds."""
-    w = cached_world("yoimiya_ground_small")
-    if w is None:
-        pytest.skip("scene cache not built")
+    w = stand_in_world("yoimiya_ground_small")
     from helpers import mesh_camera
     cam = mesh_camera((96, 64))
     rays = oracle.generate_rays(cam.to_struct(), 96, 64, 0, 3)
