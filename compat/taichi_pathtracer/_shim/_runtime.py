@@ -124,10 +124,27 @@ class ImageField:
             self.renderer.clear()
 
 
+def _devices():
+    """LPT_DEVICES: "all" or a comma list of CUDA device indices ("0,1,2,3") to split every pass over, from this one
+    process (MultiRenderer); unset renders on one device."""
+    v = os.environ.get("LPT_DEVICES", "").strip()
+    if not v:
+        return None
+    return "all" if v == "all" else [int(d) for d in v.split(",") if d.strip()]
+
+
+def _new_renderer(w, h):
+    devices = _devices()
+    if devices is None:
+        return L.Renderer(w, h, L.default_context())
+    return L.MultiRenderer(w, h, devices, L.default_context())
+
+
 def _render_pass(image, world, cam, count, depth, model, first_sample, flags=0):
-    """`count` more samples per pixel of (world, cam) into the image's device accumulator: ONE pt_render call."""
+    """`count` more samples per pixel of (world, cam) into the image's device accumulator: ONE pt_render call (one
+    pt_multi_render over the devices of LPT_DEVICES when that is set)."""
     w, h = image.shape
-    r = image.renderer or L.Renderer(w, h, L.default_context())
+    r = image.renderer or _new_renderer(w, h)
     r.render(world.device_scene(r.ctx), cam, count, depth, model, seed=int(os.environ.get("LPT_SEED", "1")),
              spp_offset=first_sample, want_stats=False, flags=flags)
     return r

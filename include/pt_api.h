@@ -249,6 +249,34 @@ int pt_postprocess_host(PtContext* ctx, const void* accum_dev, int width, int he
 /* raw device accumulator (float4[h*w]) -> host float[width][height][3]. */
 int pt_download_accum(PtContext* ctx, const void* accum_dev, int width, int height, float* out_host);
 
+/* ---- one frame on several contexts (csrc/multi.cu) ----------------------------------------- */
+typedef struct PtMulti PtMulti;
+
+/* A group of n (1..16) contexts that render one frame together.  members[0] is the ROOT: the accumulator passed to
+ * pt_multi_render lives on its device and the call is ordered on its stream.  Contexts must be distinct objects; two
+ * contexts may sit on the same device.  Enables peer access between every pair of distinct devices (an already-enabled
+ * pair is not an error); fails with PT_ERR_INVALID naming the pair when cudaDeviceCanAccessPeer says no.  The contexts
+ * stay owned by the caller and must outlive the group. */
+int pt_multi_create(PtContext* const* members, int n, PtMulti** out);
+void pt_multi_destroy(PtMulti* m);
+
+/* p->spp samples starting at p->spp_offset, split over the members exactly like multigpu.split_samples (contiguous
+ * ranges, remainder to the low members), scenes[i] rendered on members[i].  The sum over all members is ADDED into
+ * accum_root (float4[h*w] on the root's device, all 4 channels) and, with PT_FLAG_ACCUM_SQ, into accum_sq_root.
+ * The other members read and write the root's accumulators through peer access: they must be memory that peer access
+ * maps (cudaMalloc, e.g. torch's default allocator).  Every member reduces one contiguous slice of the pixels (partials
+ * of members 1, 2, ... in that order), so the result is deterministic given the per-member renders.
+ * stats == NULL: asynchronous like pt_render — returns after enqueueing; the root stream is ordered behind every member's
+ * work.  stats != NULL: stats[n], one PtStats per member; the call waits for the whole frame.
+ * Row bands (reserved[4], reserved[5]) are refused.  Every argument is checked before anything is enqueued. */
+int pt_multi_render(PtMulti* m, PtScene* const* scenes, const PtCamera* cam, const PtRenderParams* p,
+                    void* accum_root, void* accum_sq_root, PtStats* stats);
+
+/* A copy of a built scene on another context (another device or the same one): device arrays copied device to device,
+ * host staging copied, SceneView pointers rebased.  The result is the same tree, not a rebuild, and is independent of
+ * src afterwards: destroying src does not affect it, and set_* + pt_scene_build work on it as on any scene. */
+int pt_scene_replicate(const PtScene* src, PtContext* dst, PtScene** out);
+
 /* FP32 FMA peak microbenchmark (all SMs, dependent-free FMA chains): returns TFLOP/s. */
 int pt_measure_fp32_peak(PtContext* ctx, float* tflops);
 

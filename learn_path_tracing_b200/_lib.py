@@ -86,7 +86,8 @@ API_SYMBOLS = [
     "pt_scene_bvh_download", "pt_scene_triangles_download", "pt_generate_rays", "pt_trace_batch",
     "pt_trace_batch_device", "pt_random_rays_device", "pt_render", "pt_render_host", "pt_postprocess",
     "pt_postprocess_host", "pt_download_accum", "pt_measure_fp32_peak", "pt_last_error", "pt_version",
-    "pt_render_stats", "pt_build_info", "pt_generate_rays_ex",
+    "pt_render_stats", "pt_build_info", "pt_generate_rays_ex", "pt_multi_create", "pt_multi_destroy", "pt_multi_render",
+    "pt_scene_replicate",
 ]
 
 
@@ -148,6 +149,10 @@ def load():
         "pt_render_stats": (i32, [vp, P(PtStats)]),
         "pt_build_info": (C.c_char_p, []),
         "pt_generate_rays_ex": (i32, [vp, P(PtCamera), i32, i32, i32, u32, i32, vp]),
+        "pt_multi_create": (i32, [P(vp), i32, P(vp)]),
+        "pt_multi_destroy": (None, [vp]),
+        "pt_multi_render": (i32, [vp, P(vp), P(PtCamera), P(PtRenderParams), vp, vp, P(PtStats)]),
+        "pt_scene_replicate": (i32, [vp, vp, P(vp)]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)  # AttributeError if the library lacks a declared symbol
@@ -358,6 +363,15 @@ class Scene:
     def build(self):
         check(self.lib.pt_scene_build(self.handle))
 
+    def replicate(self, ctx: Context) -> "Scene":
+        """pt_scene_replicate: a copy of this built scene on `ctx` (device-to-device copies, the same tree, no rebuild);
+        independent of this scene afterwards."""
+        h = C.c_void_p()
+        check(self.lib.pt_scene_replicate(self.handle, ctx.handle, C.byref(h)))
+        out = Scene.__new__(Scene)
+        out.ctx, out.lib, out.handle = ctx, self.lib, h
+        return out
+
     def bvh_info(self):
         a, b, c = C.c_int64(), C.c_int64(), C.c_int64()
         check(self.lib.pt_scene_bvh_info(self.handle, C.byref(a), C.byref(b), C.byref(c)))
@@ -374,3 +388,44 @@ class Scene:
         tris = np.zeros((n, 12), np.float32)
         check(self.lib.pt_scene_triangles_download(self.handle, _fptr(tris), n))
         return tris
+
+
+class Multi:
+    """pt_multi_*: contexts that render one frame together.  contexts[0] is the root: the accumulators passed to render()
+    live on its device and the frame is ordered on its stream.  The contexts must outlive this object (it keeps them)."""
+
+    def __init__(self, contexts):
+        self.lib = load()
+        self.contexts = list(contexts)
+        arr = (C.c_void_p * max(len(self.contexts), 1))(*[c.handle for c in self.contexts])
+        h = C.c_void_p()
+        check(self.lib.pt_multi_create(arr, len(self.contexts), C.byref(h)))
+        self.handle = h
+
+    @property
+    def n(self) -> int:
+        return len(self.contexts)
+
+    def close(self):
+        if getattr(self, "handle", None):
+            self.lib.pt_multi_destroy(self.handle)
+            self.handle = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def render(self, scenes, cam: PtCamera, params: PtRenderParams, accum_ptr: int, accum_sq_ptr: int | None = None,
+               want_stats: bool = False) -> list[PtStats] | None:
+        """pt_multi_render: params.spp samples from params.spp_offset, split over the members, scenes[i] on member i; the sum
+        is ADDED into the root's accumulators.  want_stats=False returns None without waiting for the GPU; otherwise one
+        PtStats per member, after the whole frame."""
+        if len(scenes) != self.n:
+            raise PtError(f"pt_multi_render: {len(scenes)} scenes for {self.n} members")
+        arr = (C.c_void_p * max(len(scenes), 1))(*[s.handle for s in scenes])
+        st = (PtStats * self.n)() if want_stats else None
+        check(self.lib.pt_multi_render(self.handle, arr, C.byref(cam), C.byref(params), C.c_void_p(accum_ptr),
+                                       C.c_void_p(accum_sq_ptr or 0), st))
+        return list(st) if want_stats else None

@@ -688,18 +688,27 @@ class LegacyRenderer:
     Under an initialised torch.distributed process group (one rank per GPU) every pass of `spp` samples is split
     over the ranks (multigpu.render_split_reduce: disjoint sample ranges, scene replicated, accumulators summed onto
     rank 0 over NCCL); rank 0 owns the progressive image and returns the frame, the other ranks return None.
-    distributed=False keeps a renderer local to its rank."""
+    distributed=False keeps a renderer local to its rank.
+    devices (a list of CUDA device indices, or "all"; the first one is the context's) splits every pass over those devices
+    from this one process instead (render.MultiRenderer); it does not combine with a process group."""
 
     def __init__(self, world: World, camera: Camera, spp=32, propagate_limit=32, absorptivity=0.25, seed=1, ctx=None,
-                 distributed=True, group=None, bands=1):
-        from .render import Renderer, default_context
+                 distributed=True, group=None, bands=1, devices=None):
+        from .render import MultiRenderer, Renderer, default_context
         self.ctx = ctx or default_context()
         self.world, self.camera = world, camera
         self.spp, self.propagate_limit, self.absorptivity, self.seed = int(spp), int(propagate_limit), float(absorptivity), seed
-        self.renderer = Renderer(camera.resolution[0], camera.resolution[1], self.ctx)
-        self.frame = None
         self.group, self.bands = group, int(bands)
         self.distributed = bool(distributed)
+        if devices is not None:
+            from .multigpu import _dist_active
+            if self.distributed and _dist_active(self.group):
+                raise ValueError("LegacyRenderer: devices= splits passes within this process; with an active process group "
+                                 "pass distributed=False (or leave devices=None to split over the ranks)")
+            self.renderer = MultiRenderer(camera.resolution[0], camera.resolution[1], devices, self.ctx)
+        else:
+            self.renderer = Renderer(camera.resolution[0], camera.resolution[1], self.ctx)
+        self.frame = None
         self._total = 0       # samples per pixel in the image (over all ranks)
         self._partial = None  # ranks > 0: scratch accumulator of one pass
 

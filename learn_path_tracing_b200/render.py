@@ -58,6 +58,20 @@ class Renderer:
         want_stats=False returns None without waiting for the GPU (Renderer.stats() fetches them later).
         rows=(y0, y1) renders only that band of image rows (persistent kernel); count_samples=False leaves spp_done alone
         (all bands but the last of one banded pass)."""
+        p = self._params(spp, max_depth, shading_model, seed, spp_offset, absorptivity, flags, pool_capacity, mode,
+                         segments_per_launch, shade_min, serve_min)
+        if rows is not None:
+            p.reserved[4], p.reserved[5] = int(rows[0]), int(rows[1])
+        self.ctx.set_stream(self.torch.cuda.current_stream().cuda_stream)
+        st = self.ctx.render(scene, cam, p, self.accum.data_ptr(),
+                             self.accum_sq.data_ptr() if self.accum_sq is not None else None, want_stats=want_stats)
+        if count_samples:
+            self.spp_done += int(spp)
+        self.last_stats = st
+        return st
+
+    def _params(self, spp, max_depth, shading_model, seed, spp_offset, absorptivity, flags, pool_capacity, mode,
+                segments_per_launch, shade_min, serve_min) -> _lib.PtRenderParams:
         p = _lib.PtRenderParams()
         p.width, p.height = self.width, self.height
         p.spp = int(spp)
@@ -72,15 +86,7 @@ class Renderer:
         p.reserved[2] = int(shade_min)            # persistent: finished lanes that trigger shading/refill (0 = default)
         p.reserved[3] = int(serve_min)            # persistent: waiting lanes that trigger a service (0 = default)
         p.reserved[1] = int(segments_per_launch)  # fused: ray segments per path slot per launch (0 = 32)
-        if rows is not None:
-            p.reserved[4], p.reserved[5] = int(rows[0]), int(rows[1])
-        self.ctx.set_stream(self.torch.cuda.current_stream().cuda_stream)
-        st = self.ctx.render(scene, cam, p, self.accum.data_ptr(),
-                             self.accum_sq.data_ptr() if self.accum_sq is not None else None, want_stats=want_stats)
-        if count_samples:
-            self.spp_done += int(spp)
-        self.last_stats = st
-        return st
+        return p
 
     def side_stream(self):
         """A second CUDA stream of this renderer (reduce of one row band beside the rendering of the next)."""
@@ -110,15 +116,96 @@ class Renderer:
         return self.ctx.postprocess_host(self.accum.data_ptr(), self.width, self.height, 1.0 / n, aces, gamma)
 
 
+def resolve_devices(devices, root_device: int) -> list[int]:
+    """A device list for MultiRenderer: "all" = the root's device followed by every other visible device; otherwise the
+    given CUDA device indices (repeats allowed: two members on one device render one after the other)."""
+    if isinstance(devices, str):
+        if devices.strip() != "all":
+            raise ValueError(f"devices: 'all' or a list of CUDA device indices, not {devices!r}")
+        import torch
+        return [int(root_device)] + [d for d in range(torch.cuda.device_count()) if d != int(root_device)]
+    out = [int(d) for d in devices]
+    if not out:
+        raise ValueError("devices: empty device list")
+    return out
+
+
+def _combined_stats(stats):
+    """One PtStats for a frame rendered by several members: counts summed, time = the slowest member's."""
+    t = _lib.PtStats()
+    for s in stats:
+        for f in ("paths", "segments", "nodes_visited", "prims_tested", "launches", "launches_extend", "launches_shade"):
+            setattr(t, f, getattr(t, f) + getattr(s, f))
+        for f in ("ms_total", "ms_extend", "ms_shade", "ms_other"):
+            setattr(t, f, max(getattr(t, f), getattr(s, f)))
+        t.iterations = max(t.iterations, s.iterations)
+    t.reserved[0] = stats[0].reserved[0]
+    return t
+
+
+class MultiRenderer(Renderer):
+    """A Renderer whose frames are split over several contexts of this process (pt_multi_render): the samples of every
+    pixel are divided like multigpu.split_samples, every member renders its share on its own device and stream, and the
+    partial accumulators are summed into this renderer's accumulators on the root (member 0) by a reduce over peer
+    memory.  Member 0 is `ctx` (default: default_context()) and must sit on devices[0]; every other member is a new
+    Context on its device, bound to a torch stream of that device.  render() takes the ROOT's scene and renders replicas
+    of it on the other members (pt_scene_replicate, cached until another scene is passed)."""
+
+    def __init__(self, width: int, height: int, devices, ctx: _lib.Context | None = None, want_sq: bool = False):
+        import torch
+        root = ctx or default_context()
+        devs = resolve_devices(devices, root.device)
+        if devs[0] != root.device:
+            raise ValueError(f"devices[0] = {devs[0]} is not the root context's device {root.device}")
+        super().__init__(width, height, root, want_sq)
+        self.devices = devs
+        self.streams = [torch.cuda.Stream(device=d) for d in devs[1:]]  # kept alive with the member contexts
+        self.members = [root] + [_lib.Context(d, s.cuda_stream) for d, s in zip(devs[1:], self.streams)]
+        self.multi = _lib.Multi(self.members)
+        self.member_stats = None
+        self._source = None
+        self._replicas = None
+
+    def _scenes(self, scene: _lib.Scene):
+        if scene is not self._source:
+            self._replicas = None  # drop the replicas of the previous scene first
+            self._replicas = [scene] + [scene.replicate(c) for c in self.members[1:]]
+            self._source = scene
+        return self._replicas
+
+    def render(self, scene: _lib.Scene, cam: _lib.PtCamera, spp: int, max_depth: int,
+               shading_model: int = _lib.PT_SHADE_V2, seed: int = 1, spp_offset: int | None = None,
+               absorptivity: float = 0.25, flags: int = 0, pool_capacity: int = 0, mode: int = 0,
+               segments_per_launch: int = 0, shade_min: int = 0, serve_min: int = 0,
+               want_stats: bool = True, rows: tuple[int, int] | None = None,
+               count_samples: bool = True) -> _lib.PtStats | None:
+        """Renderer.render over all members: `spp` more samples per pixel into the root's accumulators.  want_stats=True
+        waits for the frame and returns the members' statistics combined (per member: `member_stats`)."""
+        if rows is not None:
+            raise ValueError("MultiRenderer renders whole frames: row bands (rows=) are not supported")
+        p = self._params(spp, max_depth, shading_model, seed, spp_offset, absorptivity, flags, pool_capacity, mode,
+                         segments_per_launch, shade_min, serve_min)
+        self.ctx.set_stream(self.torch.cuda.current_stream(self.accum.device).cuda_stream)
+        st = self.multi.render(self._scenes(scene), cam, p, self.accum.data_ptr(),
+                               self.accum_sq.data_ptr() if self.accum_sq is not None else None, want_stats=want_stats)
+        if count_samples:
+            self.spp_done += int(spp)
+        self.member_stats = st
+        self.last_stats = _combined_stats(st) if st else None
+        return self.last_stats
+
+
 def render(world, camera, spp: int = 8192, propagate_limit: int = 32, seed: int = 1, bsdf=None,
            ctx: _lib.Context | None = None, return_stats: bool = False, postprocess: bool = True,
-           pixel_grid: bool = False, absorptivity: float = 0.25, aces: bool = True):
+           pixel_grid: bool = False, absorptivity: float = 0.25, aces: bool = True, devices=None):
     """Drop-in for the v2 scripts' render(world, camera) + post_processing(): returns the tonemapped
-    image as a float32 [W,H,3] array in Taichi field layout (pass it to imwrite)."""
+    image as a float32 [W,H,3] array in Taichi field layout (pass it to imwrite).
+    devices: None renders on `ctx` alone; a list of CUDA device indices (or "all") splits the frame over them in this
+    process (MultiRenderer; the first device must be the context's)."""
     ctx = ctx or default_context()
     w, h = camera.resolution
     model = getattr(bsdf, "shading_model", _lib.PT_SHADE_V2)
-    r = Renderer(w, h, ctx)
+    r = Renderer(w, h, ctx) if devices is None else MultiRenderer(w, h, devices, ctx)
     st = r.render(world.device_scene(ctx), camera.to_struct(), spp, propagate_limit, model, seed, absorptivity=absorptivity,
                   flags=_lib.PT_FLAG_PIXEL_GRID if pixel_grid else 0)  # stages 2-4: lattice rays, no jitter
     img = r.image(aces=aces, gamma=2.2) if postprocess else r.mean()  # stages <= 5 write the linear image
