@@ -133,11 +133,17 @@ def _devices():
     return "all" if v == "all" else [int(d) for d in v.split(",") if d.strip()]
 
 
+def _denoise():
+    """LPT_DENOISE=1: the image is the denoised mean (Renderer.denoised(): 4-spp guide features of the first pass's camera
+    rays), as render(..., denoise=True) returns it; unset or 0 leaves the raw Monte Carlo mean."""
+    return os.environ.get("LPT_DENOISE", "").strip() not in ("", "0")
+
+
 def _new_renderer(w, h):
     devices = _devices()
     if devices is None:
-        return L.Renderer(w, h, L.default_context())
-    return L.MultiRenderer(w, h, devices, L.default_context())
+        return L.Renderer(w, h, L.default_context(), want_sq=_denoise())
+    return L.MultiRenderer(w, h, devices, L.default_context(), want_sq=_denoise())
 
 
 def _render_pass(image, world, cam, count, depth, model, first_sample, flags=0):
@@ -145,8 +151,11 @@ def _render_pass(image, world, cam, count, depth, model, first_sample, flags=0):
     pt_multi_render over the devices of LPT_DEVICES when that is set)."""
     w, h = image.shape
     r = image.renderer or _new_renderer(w, h)
-    r.render(world.device_scene(r.ctx), cam, count, depth, model, seed=int(os.environ.get("LPT_SEED", "1")),
-             spp_offset=first_sample, want_stats=False, flags=flags)
+    seed = int(os.environ.get("LPT_SEED", "1"))
+    scene = world.device_scene(r.ctx)
+    r.render(scene, cam, count, depth, model, seed=seed, spp_offset=first_sample, want_stats=False, flags=flags)
+    if _denoise() and first_sample == 0:
+        r.features(scene, cam, 4, seed, 0, flags, model)
     return r
 
 
@@ -155,7 +164,9 @@ def _read_image(image):
     if image.renderer is None:
         return np.zeros((w, h, 3), np.float32)
     if image.post is not None:
-        return image.renderer.image(aces=image.post[0], gamma=image.post[1], total_spp=image.norm)
+        return image.renderer.image(aces=image.post[0], gamma=image.post[1], total_spp=image.norm, denoise=_denoise())
+    if _denoise():
+        return L.denoised_mean(image.renderer, total_spp=image.norm)
     return image.renderer.ctx.download_accum(image.renderer.accum.data_ptr(), w, h) / np.float32(image.norm)
 
 

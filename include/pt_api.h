@@ -17,6 +17,7 @@
  *   pt_render[_host]            render(): get_rays + shader loop    10_final/__main__.py:78-87,99-103
  *                               render(): get_rays + propagate_once + gen_secondary_rays   15_module.py:980-1036
  *   pt_postprocess[_host]       post_processing / gamma_correction  10_final/__main__.py:90-96, 15_module.py:1016-1019
+ *   pt_render_features, pt_denoise   (no reference counterpart: an opt-in denoised mean of a low-sample frame)
  *
  * Conventions
  *   - every function returns 0 on success, a negative PT_ERR_* otherwise; pt_last_error() returns
@@ -276,6 +277,34 @@ int pt_multi_render(PtMulti* m, PtScene* const* scenes, const PtCamera* cam, con
  * host staging copied, SceneView pointers rebased.  The result is the same tree, not a rebuild, and is independent of
  * src afterwards: destroying src does not affect it, and set_* + pt_scene_build work on it as on any scene. */
 int pt_scene_replicate(const PtScene* src, PtContext* dst, PtScene** out);
+
+/* ---- denoising (csrc/denoise.cu) ---------------------------------------------------------- */
+/* First-hit guide features of the camera rays of samples [p->spp_offset, p->spp_offset + p->spp) of every pixel: the
+ * same rays pt_render starts its paths with (rng4(pixel, sample, 0, seed), PT_FLAG_PIXEL_GRID honoured), hit with
+ * the same acceptance rule (tmin of the shading model).  ADDED into features_dev = float4[2][h*w] (pixel j*w + i,
+ * j up, like the accumulator); the caller zeroes it, so passes and progressive poses compose like accum_dev:
+ *   plane 0: sum over hits of (shading normal turned to face the ray).xyz, hit distance t
+ *   plane 1: sum over ALL samples of albedo.rgb, and the number of hits in .w
+ * A miss adds 0 to plane 0 and the miss radiance clamped to [0,1] (sky gradient / environment) as its albedo.
+ * Accepts and refuses what pt_render does for the same scene and parameters, except: row bands (reserved[4..5]) are
+ * refused, the mode / threshold fields reserved[0..3] are ignored, PT_FLAG_ACCUM_SQ needs no buffer.
+ * Asynchronous on the context stream. */
+int pt_render_features(PtContext* ctx, const PtScene* s, const PtCamera* cam, const PtRenderParams* p,
+                       void* features_dev);
+
+typedef struct PtDenoiseParams {
+    int32_t width, height;
+    int32_t spp;          /* samples per pixel in accum (the mean is accum / spp, as pt_postprocess's scale)  */
+    int32_t iterations;   /* a-trous passes, 0..10 (0 = no filtering: out = accum / spp)                      */
+    float sigma_l, sigma_n, sigma_z;   /* edge-stopping strengths; 0 = defaults 4, 128, 1                  */
+    int32_t _pad;
+} PtDenoiseParams; /* 32 bytes */
+
+/* Denoised mean radiance into out_dev = float4[h*w] (rgb, w = 1), ready for pt_postprocess with scale 1.
+ * Needs the sum of squares (PT_FLAG_ACCUM_SQ) and a feature buffer of the same size. Deterministic: no atomics.
+ * Every argument is checked before anything is enqueued.  Asynchronous on the context stream. */
+int pt_denoise(PtContext* ctx, const void* accum_dev, const void* accum_sq_dev, const void* features_dev,
+               const PtDenoiseParams* p, void* out_dev);
 
 /* FP32 FMA peak microbenchmark (all SMs, dependent-free FMA chains): returns TFLOP/s. */
 int pt_measure_fp32_peak(PtContext* ctx, float* tflops);

@@ -70,7 +70,12 @@ class PtStats(C.Structure):
         return {n: getattr(self, n) for n, _ in self._fields_ if n != "reserved"}
 
 
-assert C.sizeof(PtMaterial) == 32 and C.sizeof(PtCamera) == 64
+class PtDenoiseParams(C.Structure):
+    _fields_ = [("width", C.c_int32), ("height", C.c_int32), ("spp", C.c_int32), ("iterations", C.c_int32),
+                ("sigma_l", C.c_float), ("sigma_n", C.c_float), ("sigma_z", C.c_float), ("_pad", C.c_int32)]
+
+
+assert C.sizeof(PtMaterial) == 32 and C.sizeof(PtCamera) == 64 and C.sizeof(PtDenoiseParams) == 32
 assert C.sizeof(PtRenderParams) == 64 and C.sizeof(PtStats) == 80
 
 MATERIAL_DTYPE = np.dtype([("albedo", "<f4", 3), ("roughness", "<f4"), ("metallic", "<i4"), ("ior", "<f4"),
@@ -87,7 +92,7 @@ API_SYMBOLS = [
     "pt_trace_batch_device", "pt_random_rays_device", "pt_render", "pt_render_host", "pt_postprocess",
     "pt_postprocess_host", "pt_download_accum", "pt_measure_fp32_peak", "pt_last_error", "pt_version",
     "pt_render_stats", "pt_build_info", "pt_generate_rays_ex", "pt_multi_create", "pt_multi_destroy", "pt_multi_render",
-    "pt_scene_replicate",
+    "pt_scene_replicate", "pt_render_features", "pt_denoise",
 ]
 
 
@@ -153,6 +158,8 @@ def load():
         "pt_multi_destroy": (None, [vp]),
         "pt_multi_render": (i32, [vp, P(vp), P(PtCamera), P(PtRenderParams), vp, vp, P(PtStats)]),
         "pt_scene_replicate": (i32, [vp, vp, P(vp)]),
+        "pt_render_features": (i32, [vp, vp, P(PtCamera), P(PtRenderParams), vp]),
+        "pt_denoise": (i32, [vp, vp, vp, vp, P(PtDenoiseParams), vp]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)  # AttributeError if the library lacks a declared symbol
@@ -258,6 +265,19 @@ class Context:
         st = PtStats()
         check(self.lib.pt_render_stats(self.handle, C.byref(st)))
         return st
+
+    def render_features(self, scene: "Scene", cam: PtCamera, params: PtRenderParams, features_ptr: int):
+        """pt_render_features: first-hit normal / depth / albedo of samples [spp_offset, spp_offset + spp) ADDED into
+        features_ptr (float4[2][h*w]); asynchronous on the context's stream."""
+        check(self.lib.pt_render_features(self.handle, scene.handle, C.byref(cam), C.byref(params), C.c_void_p(features_ptr)))
+
+    def denoise(self, accum_ptr: int, accum_sq_ptr: int | None, features_ptr: int, width: int, height: int, spp: int,
+                out_ptr: int, iterations: int = 5, sigma_l: float = 0.0, sigma_n: float = 0.0, sigma_z: float = 0.0):
+        """pt_denoise: the denoised mean radiance (float4[h*w], w = 1) into out_ptr; asynchronous on the context's stream."""
+        p = PtDenoiseParams(int(width), int(height), int(spp), int(iterations), float(sigma_l), float(sigma_n),
+                            float(sigma_z), 0)
+        check(self.lib.pt_denoise(self.handle, C.c_void_p(accum_ptr), C.c_void_p(accum_sq_ptr or 0),
+                                  C.c_void_p(features_ptr), C.byref(p), C.c_void_p(out_ptr)))
 
     def render_host(self, scene: "Scene", cam: PtCamera, params: PtRenderParams, want_sq: bool = False):
         W, H = params.width, params.height

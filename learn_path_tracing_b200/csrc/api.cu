@@ -67,6 +67,7 @@ extern "C" void pt_context_destroy(PtContext* c) {
     if (c->hits) cudaFree(c->hits);
     if (c->scratch) cudaFree(c->scratch);
     if (c->sort_scratch) cudaFree(c->sort_scratch);
+    if (c->px_scratch) cudaFree(c->px_scratch);
     for (int b = 0; b < 2; ++b) {
         if (c->stage_rays_h[b]) cudaFreeHost(c->stage_rays_h[b]);
         if (c->stage_hits_h[b]) cudaFreeHost(c->stage_hits_h[b]);

@@ -94,6 +94,10 @@ struct PtContext {
     // grow-only device scratch for host-layout read-backs (no cudaMalloc/cudaFree on the render path)
     void* scratch = nullptr;
     size_t scratch_bytes = 0;
+    // grow-only device scratch of the denoiser, 48 B per pixel (denoise.cu): camera rays + hits of one sample in
+    // pt_render_features, colour ping-pong + guides in pt_denoise.  Apart from `scratch`, which pt_download_accum reallocates
+    void* px_scratch = nullptr;
+    size_t px_scratch_bytes = 0;
     // grow-only device scratch of the ray sort (keys, order, cub temporaries)
     void* sort_scratch = nullptr;
     size_t sort_bytes = 0;
@@ -189,3 +193,10 @@ int pt_render_queue(PtContext* ctx, const PtScene* s, const RenderConsts& rc, bo
                     float4* accum_sq, int serve_min);
 // post.cu
 int pt_ensure_scratch(PtContext* ctx, size_t bytes);
+// wavefront.cu — pt_render's argument checks (features = true: pt_render_features' variant), the hit acceptance of a shading
+// model, and the first hits of the camera rays of one sample (rays float4[2 W H], hits float4[W H], asynchronous)
+int pt_check_render_args(const char* fn, const PtContext* ctx, const PtScene* s, const PtCamera* cam, const PtRenderParams* p,
+                         const void* accum_dev, const void* accum_sq_dev, bool features);
+float pt_render_tmin(int shading_model);
+int pt_first_hits(PtContext* ctx, const PtScene* s, const PtCamera* cam, int W, int H, int flags, uint32_t sample,
+                  uint32_t seed, float tmin, float4* rays, float4* hits);

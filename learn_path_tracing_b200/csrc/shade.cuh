@@ -54,6 +54,13 @@ PT_DEV float3 refract_dir(float3 d, float3 n, float ior) {  // bsdf.py:47-59
     return perp - sqrtf(1.0f - len2) * n;
 }
 
+// ---- surface attributes at a hit ----------------------------------------------------------------
+// The scatter code and the denoiser's first-hit features (denoise.cu) read a surface through these, so both see the
+// same normal and albedo.  Outward normals: the caller turns them to face the ray.
+PT_DEV float3 sphere_normal_v2(float4 cr, float3 point) {  // world.py:58
+    return normalize(point - f3(cr));
+}
+
 // ---- v2 scatter: one propagate_once hit branch (__main__.py:65-75) -----------------------------
 // mat0 = albedo.rgb, roughness ; mat1 = bits(metallic), ior, bits(transparency), _
 PT_DEV void scatter_v2(const SceneView& sv, PathState& p, const Hit& h, int shading_model, uint32_t seed) {
@@ -62,7 +69,7 @@ PT_DEV void scatter_v2(const SceneView& sv, PathState& p, const Hit& h, int shad
     const float4 m1 = __ldg(&sv.sph_mat[2 * h.prim + 1]);
     const float3 albedo = f3(m0);
     const float3 point = p.o + h.t * p.d;            // world.py:57
-    float3 normal = normalize(point - f3(cr));       // world.py:58
+    float3 normal = sphere_normal_v2(cr, point);
     float ior = m1.y;
     if (dot(p.d, normal) > 0.0f) {                   // world.py:31-33
         normal = -normal;
@@ -267,14 +274,14 @@ PT_DEV float3 sample_in_sphere(float u0, float u1, float u2) {  // 15_module.py:
     return f3(r * ct * sphi, r * st * sphi, r * cphi);
 }
 
-// propagate_once hit branch (15_module.py:983-989) + gen_secondary_rays (:994-1013)
-PT_DEV void scatter_legacy(const SceneView& sv, PathState& p, const Hit& h, float absorptivity, uint32_t seed,
-                           const float* lut) {
-    const float3 d = p.d;
-    const float3 point = p.o + h.t * d;
-    float3 normal, albedo;
-    float roughness, metallic, ior = 1.5f;
-    int transparency = 0;
+struct LegacySurface {
+    float3 normal, albedo;  // outward shading normal (normal-mapped on spheres), texture albedo
+    float roughness, metallic;
+    int transparency;
+};
+PT_DEV LegacySurface legacy_surface(const SceneView& sv, const float* lut, const Hit& h, float3 point) {
+    LegacySurface o;
+    o.transparency = 0;
     if (h.prim < sv.n_sph) {  // sphere_hit, 15_module.py:864-896
         const float4 cr = __ldg(&sv.sph_cr[h.prim]);
         const float4 aux = __ldg(&sv.sph_aux[h.prim]);
@@ -287,19 +294,33 @@ PT_DEV void scatter_legacy(const SceneView& sv, PathState& p, const Hit& h, floa
         const float uu = (theta * (1.0f / PT_PI) + 1.0f) * 0.5f;
         const float vv = phi * (1.0f / PT_PI) + 0.5f;
         const Texel tx = sample_texture(sv, lut, __float_as_int(aux.z), 2.0f * uu, vv, true);
-        normal = normalize(tx.normal.x * T + tx.normal.y * B + tx.normal.z * N);
-        albedo = tx.albedo; roughness = tx.roughness; metallic = tx.metallic;
-        transparency = __float_as_int(aux.y);
+        o.normal = normalize(tx.normal.x * T + tx.normal.y * B + tx.normal.z * N);
+        o.albedo = tx.albedo; o.roughness = tx.roughness; o.metallic = tx.metallic;
+        o.transparency = __float_as_int(aux.y);
     } else {  // triangle_hit, 15_module.py:929-950
         const float4* s = sv.tri_shade + 4 * (size_t)(h.prim - sv.n_sph);
         const float4 s0 = __ldcg(s), s1 = __ldcg(s + 1), s2 = __ldcg(s + 2), s3 = __ldcg(s + 3);
         const float w1 = 1.0f - h.u - h.v, w2 = h.u, w3 = h.v;
-        normal = normalize(w1 * f3(s0) + w2 * f3(s1) + w3 * f3(s2));
+        o.normal = normalize(w1 * f3(s0) + w2 * f3(s1) + w3 * f3(s2));
         const float uu = w1 * s0.w + w2 * s2.w + w3 * s3.y;
         const float vv = w1 * s1.w + w2 * s3.x + w3 * s3.z;
         const Texel tx = sample_texture(sv, lut, __float_as_int(s3.w), uu, vv, false);
-        albedo = tx.albedo; roughness = tx.roughness; metallic = tx.metallic;
+        o.albedo = tx.albedo; o.roughness = tx.roughness; o.metallic = tx.metallic;
     }
+    return o;
+}
+
+// propagate_once hit branch (15_module.py:983-989) + gen_secondary_rays (:994-1013)
+PT_DEV void scatter_legacy(const SceneView& sv, PathState& p, const Hit& h, float absorptivity, uint32_t seed,
+                           const float* lut) {
+    const float3 d = p.d;
+    const float3 point = p.o + h.t * d;
+    const LegacySurface sf = legacy_surface(sv, lut, h, point);
+    float3 normal = sf.normal;
+    const float3 albedo = sf.albedo;
+    const float roughness = sf.roughness, metallic = sf.metallic;
+    const int transparency = sf.transparency;
+    float ior = 1.5f;
     if (dot(d, normal) > 0.0f) {  // 15_module.py:985-988
         normal = -normal;
         ior = 1.0f / ior;

@@ -267,12 +267,12 @@ k_trace(const SceneView sv, const float4* __restrict__ rays, float4* __restrict_
     }
 }
 
-__global__ void k_generate_rays(const CameraDev cam, int W, int H, uint32_t sample, uint32_t seed, float4* rays) {
+__global__ void k_generate_rays(const CameraDev cam, int W, int H, uint32_t sample, uint32_t seed, float tmin, float4* rays) {
     const unsigned pix = blockIdx.x * blockDim.x + threadIdx.x;
     if (pix >= (unsigned)W * (unsigned)H) return;
     float3 o, d;
     camera_ray(cam, (int)(pix % (unsigned)W), (int)(pix / (unsigned)W), rng4(pix, sample, 0u, seed), &o, &d);
-    rays[2 * pix] = make_float4(o.x, o.y, o.z, PT_EPS);
+    rays[2 * pix] = make_float4(o.x, o.y, o.z, tmin);
     rays[2 * pix + 1] = make_float4(d.x, d.y, d.z, INFINITY);
 }
 
@@ -436,40 +436,79 @@ static int render_fused(PtContext* ctx, const PtScene* s, const RenderConsts& rc
     return PT_OK;
 }
 
-extern "C" int pt_render(PtContext* ctx, const PtScene* s, const PtCamera* cam, const PtRenderParams* p,
-                         void* accum_dev, void* accum_sq_dev, PtStats* stats) {
-    PT_REQUIRE(ctx && s && cam && p && accum_dev, "null argument");
-    if (!s->built) { pt_set_error("pt_render: scene not built"); return PT_ERR_NOT_BUILT; }
-    PT_REQUIRE(p->width > 0 && p->height > 0 && p->spp >= 0, "bad image size / spp");
-    PT_REQUIRE(p->max_depth > 0 && p->max_depth < 256, "max_depth must be in [1,255]");
-    PT_REQUIRE((long long)p->spp_offset + p->spp <= (1 << 24), "sample index must stay below 2^24");
-    PT_REQUIRE((long long)p->width * p->height < (1ll << 31), "image too large");
-    PT_REQUIRE(p->shading_model >= 0 && p->shading_model <= 5, "unknown shading model");
+// Argument checks of pt_render, shared with pt_render_features (features = true: there is no sum-of-squares buffer, the
+// mode / threshold fields reserved[0..3] are ignored and row bands are refused).  Errors name `fn`.
+#define PT_REQUIRE_FN(cond, msg)                     \
+    do {                                             \
+        if (!(cond)) {                               \
+            pt_set_error("%s: %s", fn, msg);         \
+            return PT_ERR_INVALID;                   \
+        }                                            \
+    } while (0)
+int pt_check_render_args(const char* fn, const PtContext* ctx, const PtScene* s, const PtCamera* cam, const PtRenderParams* p,
+                         const void* accum_dev, const void* accum_sq_dev, bool features) {
+    PT_REQUIRE_FN(ctx && s && cam && p && accum_dev, "null argument");
+    if (!s->built) { pt_set_error("%s: scene not built", fn); return PT_ERR_NOT_BUILT; }
+    PT_REQUIRE_FN(p->width > 0 && p->height > 0 && p->spp >= 0, "bad image size / spp");
+    PT_REQUIRE_FN(p->max_depth > 0 && p->max_depth < 256, "max_depth must be in [1,255]");
+    PT_REQUIRE_FN((long long)p->spp_offset + p->spp <= (1 << 24), "sample index must stay below 2^24");
+    PT_REQUIRE_FN((long long)p->width * p->height < (1ll << 31), "image too large");
+    PT_REQUIRE_FN(p->shading_model >= 0 && p->shading_model <= 5, "unknown shading model");
     const bool legacy = p->shading_model == PT_SHADE_LEGACY;
-    PT_REQUIRE(legacy || (s->view.n_tri == 0 && !s->view.legacy_spheres), "v2 shading models need a v2 sphere scene");
-    PT_REQUIRE(!legacy || s->view.n_sph == 0 || s->view.legacy_spheres, "legacy shading needs legacy (textured) spheres");
-    PT_REQUIRE(!(p->flags & PT_FLAG_PIXEL_GRID) || (p->width >= 2 && p->height >= 2), "PT_FLAG_PIXEL_GRID needs width, height >= 2");
+    PT_REQUIRE_FN(legacy || (s->view.n_tri == 0 && !s->view.legacy_spheres), "v2 shading models need a v2 sphere scene");
+    PT_REQUIRE_FN(!legacy || s->view.n_sph == 0 || s->view.legacy_spheres, "legacy shading needs legacy (textured) spheres");
+    PT_REQUIRE_FN(!(p->flags & PT_FLAG_PIXEL_GRID) || (p->width >= 2 && p->height >= 2), "PT_FLAG_PIXEL_GRID needs width, height >= 2");
     const bool want_sq = (p->flags & PT_FLAG_ACCUM_SQ) != 0;
-    PT_REQUIRE(!want_sq || accum_sq_dev, "PT_FLAG_ACCUM_SQ needs accum_sq");
-    PT_REQUIRE(p->reserved[0] >= 0 && p->reserved[0] <= 5, "reserved[0] (wavefront mode) must be 0 ... 5");
-    PT_REQUIRE(p->reserved[1] >= 0 && p->reserved[1] <= 4096, "reserved[1] (segments per launch) out of range");
-    PT_REQUIRE(p->reserved[2] >= 0 && p->reserved[2] <= 32 && p->reserved[3] >= 0 && p->reserved[3] <= 32,
-               "reserved[2]/[3] (persistent-mode lane thresholds) must be in [0,32]");
+    PT_REQUIRE_FN(features || !want_sq || accum_sq_dev, "PT_FLAG_ACCUM_SQ needs accum_sq");
+    if (!features) {
+        PT_REQUIRE_FN(p->reserved[0] >= 0 && p->reserved[0] <= 5, "reserved[0] (wavefront mode) must be 0 ... 5");
+        PT_REQUIRE_FN(p->reserved[1] >= 0 && p->reserved[1] <= 4096, "reserved[1] (segments per launch) out of range");
+        PT_REQUIRE_FN(p->reserved[2] >= 0 && p->reserved[2] <= 32 && p->reserved[3] >= 0 && p->reserved[3] <= 32,
+                      "reserved[2]/[3] (persistent-mode lane thresholds) must be in [0,32]");
+    }
     // auto: the persistent ballot-scheduled kernel (measured faster than the K-step fused wavefront on every
     // workload, tree-less scenes included: 16.3 vs 15.3 Gpaths/s on 8_refract 1080p)
-    const int mode = p->reserved[0] != PT_MODE_AUTO ? p->reserved[0] : PT_MODE_PERSIST;
-    PT_REQUIRE(p->shading_model != PT_SHADE_V2_NORMALS || mode >= PT_MODE_PERSIST,
-               "PT_SHADE_V2_NORMALS needs a persistent kernel (mode 0, 3, 4 or 5)");
+    const int mode = !features && p->reserved[0] != PT_MODE_AUTO ? p->reserved[0] : PT_MODE_PERSIST;
+    PT_REQUIRE_FN(p->shading_model != PT_SHADE_V2_NORMALS || mode >= PT_MODE_PERSIST,
+                  "PT_SHADE_V2_NORMALS needs a persistent kernel (mode 0, 3, 4 or 5)");
     const bool stage = p->shading_model == PT_SHADE_LEGACY_STAGE6 || p->shading_model == PT_SHADE_LEGACY_STAGE7;
-    PT_REQUIRE(!stage || mode == PT_MODE_PERSIST, "PT_SHADE_LEGACY_STAGE6/7 need the persistent kernel (mode 0 or 3)");
+    PT_REQUIRE_FN(!stage || mode == PT_MODE_PERSIST, "PT_SHADE_LEGACY_STAGE6/7 need the persistent kernel (mode 0 or 3)");
+    const bool banded = p->reserved[4] != 0 || p->reserved[5] != 0;
+    PT_REQUIRE_FN(!features || !banded, "row bands (reserved[4], reserved[5]) are not supported");
+    PT_REQUIRE_FN(!banded || (p->reserved[4] >= 0 && p->reserved[4] < p->reserved[5] && p->reserved[5] <= p->height),
+                  "reserved[4]/[5] (row band) must satisfy 0 <= row0 < row1 <= height");
+    PT_REQUIRE_FN(!banded || mode == PT_MODE_PERSIST, "row bands need the persistent kernel (mode 0 or 3)");
+#ifndef PT_EXPERIMENTAL
+    PT_REQUIRE_FN(mode != PT_MODE_QUEUE && mode != PT_MODE_DUAL,
+                  "render modes 4 (queue) and 5 (dual) are experimental kernel forms: rebuild with `make EXPERIMENTAL=1`");
+#endif
+    PT_REQUIRE_FN(mode != PT_MODE_PERSIST || !(p->flags & PT_FLAG_WIDE) || s->view.wnodes,
+                  "PT_FLAG_WIDE: the scene has no 4-wide tree (build it with PT_WIDE=1 in the environment)");
+    return PT_OK;
+}
+#undef PT_REQUIRE_FN
+
+// closest-hit acceptance of a shading model: legacy accepts t > eps, v2 t >= 1e-4, the legacy tutorial stages
+// record.t > 1e-3 (7_reflect.py:148)
+float pt_render_tmin(int shading_model) {
+    if (shading_model == PT_SHADE_LEGACY_STAGE6 || shading_model == PT_SHADE_LEGACY_STAGE7) return nextafterf(1e-3f, 1.0f);
+    return shading_model == PT_SHADE_LEGACY ? nextafterf(PT_EPS, 1.0f) : PT_EPS;
+}
+
+extern "C" int pt_render(PtContext* ctx, const PtScene* s, const PtCamera* cam, const PtRenderParams* p,
+                         void* accum_dev, void* accum_sq_dev, PtStats* stats) {
+    {
+        const int rca = pt_check_render_args("pt_render", ctx, s, cam, p, accum_dev, accum_sq_dev, false);
+        if (rca) return rca;
+    }
+    const bool legacy = p->shading_model == PT_SHADE_LEGACY;
+    const bool want_sq = (p->flags & PT_FLAG_ACCUM_SQ) != 0;
+    const int mode = p->reserved[0] != PT_MODE_AUTO ? p->reserved[0] : PT_MODE_PERSIST;
     PT_CUDA(cudaSetDevice(ctx->device));
 
     // reserved[4], [5]: a band of rows [row0, row1) instead of the whole frame (0, 0 = all rows) — the multi-GPU path
     // renders band by band so that the reduce of one band overlaps the rendering of the next (persistent kernel only)
     const bool banded = p->reserved[4] != 0 || p->reserved[5] != 0;
-    PT_REQUIRE(!banded || (p->reserved[4] >= 0 && p->reserved[4] < p->reserved[5] && p->reserved[5] <= p->height),
-               "reserved[4]/[5] (row band) must satisfy 0 <= row0 < row1 <= height");
-    PT_REQUIRE(!banded || mode == PT_MODE_PERSIST, "row bands need the persistent kernel (mode 0 or 3)");
     const int row0 = banded ? p->reserved[4] : 0, row1 = banded ? p->reserved[5] : p->height;
     const unsigned long long total = (unsigned long long)p->width * (unsigned long long)(row1 - row0) * (unsigned long long)p->spp;
     const size_t def_cap = mode == PT_MODE_SPLIT ? (size_t)1 << 22 : (size_t)1 << 21;
@@ -487,8 +526,7 @@ extern "C" int pt_render(PtContext* ctx, const PtScene* s, const PtCamera* cam, 
     rc.seed = p->seed; rc.spp_offset = (uint32_t)p->spp_offset;
     rc.max_depth = p->max_depth; rc.shading_model = p->shading_model;
     rc.absorptivity = p->absorptivity;
-    rc.tmin = legacy ? nextafterf(PT_EPS, 1.0f) : PT_EPS;  // legacy accepts t > eps, v2 t >= 1e-4
-    if (stage) rc.tmin = nextafterf(1e-3f, 1.0f);          // legacy tutorial stages: record.t > 1e-3 (7_reflect.py:148)
+    rc.tmin = pt_render_tmin(p->shading_model);
     rc.pool_cap = (unsigned)cap;
     rc.accum_sq = want_sq ? 1 : 0;
     const unsigned long long WH = (unsigned long long)p->width * p->height;
@@ -516,10 +554,6 @@ extern "C" int pt_render(PtContext* ctx, const PtScene* s, const PtCamera* cam, 
 
     int iterations = 0, launches = 0, rcode;
     size_t ev_idx = 0;
-#ifndef PT_EXPERIMENTAL
-    PT_REQUIRE(mode != PT_MODE_QUEUE && mode != PT_MODE_DUAL,
-               "render modes 4 (queue) and 5 (dual) are experimental kernel forms: rebuild with `make EXPERIMENTAL=1`");
-#endif
     if (mode == PT_MODE_QUEUE) {
 #ifdef PT_EXPERIMENTAL
         const int serve_min = p->reserved[3] > 0 ? p->reserved[3] : 24;
@@ -553,7 +587,6 @@ extern "C" int pt_render(PtContext* ctx, const PtScene* s, const PtCamera* cam, 
         const int serve_min = p->reserved[3] > 0 ? p->reserved[3] : (legacy ? 8 : 12);
         if (timing) cudaEventRecord(get_event(ctx, ev_idx++), st);
         const bool wide = (p->flags & PT_FLAG_WIDE) != 0;
-        PT_REQUIRE(!wide || s->view.wnodes, "PT_FLAG_WIDE: the scene has no 4-wide tree (build it with PT_WIDE=1 in the environment)");
         rcode = pt_render_persist(ctx, s, rc, legacy, count, (float4*)accum_dev, (float4*)accum_sq_dev, shade_min, serve_min, wide);
         if (timing) cudaEventRecord(get_event(ctx, ev_idx++), st);
         iterations = 1; launches = 1;
@@ -633,6 +666,46 @@ extern "C" int pt_render_stats(PtContext* ctx, PtStats* stats) {
 }
 
 // ------------------------------------------------------------------------------------------------
+// The tracer of pt_trace_batch_device for n > 0 rays (counters zeroed by the caller): one ray per thread without a tree
+// or with PT_FLAG_TRACE_SIMPLE, else the persistent while-while warps over the (sorted) batch.
+static int trace_dispatch(PtContext* ctx, const PtScene* s, const float4* rays, long long n, float4* hits, int flags, bool count,
+                          cudaEvent_t ev_sorted, bool* persist) {
+    cudaStream_t st = ctx->stream;
+    *persist = false;
+    if ((flags & PT_FLAG_TRACE_SIMPLE) || s->view.root == PT_NO_BVH) {  // one ray per thread, batch order
+        const unsigned blocks = (unsigned)((n + PT_BLOCK - 1) / PT_BLOCK);
+        if (count) k_trace<true><<<blocks, PT_BLOCK, 0, st>>>(s->view, rays, hits, n, ctx->counters);
+        else k_trace<false><<<blocks, PT_BLOCK, 0, st>>>(s->view, rays, hits, n, ctx->counters);
+        return PT_OK;
+    }
+    const bool sort = !(flags & PT_FLAG_NO_SORT) && n >= (1 << 16);
+    const int serve_min = (flags >> 8) & 63, fetch_min = (flags >> 14) & 63;
+    const bool wide = (flags & PT_FLAG_TRACE_WIDE) != 0;
+    if (wide && !s->view.wnodes) {
+        pt_set_error("pt_trace_batch_device: PT_FLAG_TRACE_WIDE: the scene has no 4-wide tree (build it with PT_WIDE=1 in the environment)");
+        return PT_ERR_INVALID;
+    }
+    const int rct = pt_trace_persist(ctx, s, rays, n, hits, count, sort, !(flags & PT_FLAG_NO_QNODES), serve_min ? serve_min : 8,
+                                     fetch_min ? fetch_min : 8, ev_sorted, wide);
+    if (rct) return rct;
+    *persist = true;
+    return PT_OK;
+}
+
+// Camera rays of one sample of every pixel into rays (float4[2 * W * H], pt_trace_batch_device layout) and their closest
+// hits into hits (float4[W * H]), asynchronously on the context stream: the first-hit pass of pt_render_features.
+int pt_first_hits(PtContext* ctx, const PtScene* s, const PtCamera* cam, int W, int H, int flags, uint32_t sample,
+                  uint32_t seed, float tmin, float4* rays, float4* hits) {
+    cudaStream_t st = ctx->stream;
+    const long long n = (long long)W * H;
+    k_generate_rays<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(make_camera(cam, W, H, (flags & PT_FLAG_PIXEL_GRID) ? 1 : 0),
+                                                                 W, H, sample, seed, tmin, rays);
+    PT_CUDA(cudaMemsetAsync(ctx->counters, 0, CNT_WORDS * sizeof(unsigned long long), st));
+    bool persist;
+    // camera rays in pixel order are coherent already: no sort
+    return trace_dispatch(ctx, s, rays, n, hits, PT_FLAG_NO_SORT, false, nullptr, &persist);
+}
+
 extern "C" int pt_trace_batch_device(PtContext* ctx, const PtScene* s, const void* rays_dev, int64_t n,
                                      void* hits_dev, int flags, PtStats* stats) {
     PT_REQUIRE(ctx && s && (n == 0 || (rays_dev && hits_dev)), "null argument");
@@ -647,20 +720,9 @@ extern "C" int pt_trace_batch_device(PtContext* ctx, const PtScene* s, const voi
     PT_CUDA(cudaMemsetAsync(ctx->counters, 0, CNT_WORDS * sizeof(unsigned long long), st));
     PT_CUDA(cudaEventRecord(ctx->ev_a, st));
     if (n > 0) {
-        if ((flags & PT_FLAG_TRACE_SIMPLE) || s->view.root == PT_NO_BVH) {  // one ray per thread, batch order
-            const unsigned blocks = (unsigned)((n + PT_BLOCK - 1) / PT_BLOCK);
-            if (count) k_trace<true><<<blocks, PT_BLOCK, 0, st>>>(s->view, (const float4*)rays_dev, (float4*)hits_dev, n, ctx->counters);
-            else k_trace<false><<<blocks, PT_BLOCK, 0, st>>>(s->view, (const float4*)rays_dev, (float4*)hits_dev, n, ctx->counters);
-        } else {  // persistent while-while warps over the (sorted) batch
-            const bool sort = !(flags & PT_FLAG_NO_SORT) && n >= (1 << 16);
-            const int serve_min = (flags >> 8) & 63, fetch_min = (flags >> 14) & 63;
-            const bool wide = (flags & PT_FLAG_TRACE_WIDE) != 0;
-            PT_REQUIRE(!wide || s->view.wnodes, "PT_FLAG_TRACE_WIDE: the scene has no 4-wide tree (build it with PT_WIDE=1 in the environment)");
-            int rct = pt_trace_persist(ctx, s, (const float4*)rays_dev, n, (float4*)hits_dev, count, sort, !(flags & PT_FLAG_NO_QNODES),
-                                       serve_min ? serve_min : 8, fetch_min ? fetch_min : 8, stats ? get_event(ctx, 0) : nullptr, wide);
-            if (rct) return rct;
-            persist = true;
-        }
+        const int rct = trace_dispatch(ctx, s, (const float4*)rays_dev, n, (float4*)hits_dev, flags, count,
+                                       stats ? get_event(ctx, 0) : nullptr, &persist);
+        if (rct) return rct;
     }
     PT_CUDA(cudaEventRecord(ctx->ev_b, st));
     PT_CUDA(cudaGetLastError());
@@ -708,7 +770,7 @@ extern "C" int pt_generate_rays_ex(PtContext* ctx, const PtCamera* cam, int widt
     float4* d = nullptr;
     PT_CUDA(cudaMalloc(&d, n * 2 * sizeof(float4)));
     k_generate_rays<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(make_camera(cam, width, height, lattice), width, height,
-                                                                         (uint32_t)sample, seed, d);
+                                                                         (uint32_t)sample, seed, PT_EPS, d);
     cudaError_t e = cudaMemcpyAsync(rays_host, d, n * 2 * sizeof(float4), cudaMemcpyDeviceToHost, ctx->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
     cudaFree(d);

@@ -690,24 +690,34 @@ class LegacyRenderer:
     rank 0 over NCCL); rank 0 owns the progressive image and returns the frame, the other ranks return None.
     distributed=False keeps a renderer local to its rank.
     devices (a list of CUDA device indices, or "all"; the first one is the context's) splits every pass over those devices
-    from this one process instead (render.MultiRenderer); it does not combine with a process group."""
+    from this one process instead (render.MultiRenderer); it does not combine with a process group.
+    denoise=True returns denoised frames (Renderer.denoised()): the guide features of a pose are computed once, when the
+    image restarts (render(moved=True)), and serve every progressive pass of that pose.  The process-group path reduces
+    RGB only, not the sum of squares the filter needs, so denoise=True refuses an active process group."""
 
     def __init__(self, world: World, camera: Camera, spp=32, propagate_limit=32, absorptivity=0.25, seed=1, ctx=None,
-                 distributed=True, group=None, bands=1, devices=None):
+                 distributed=True, group=None, bands=1, devices=None, denoise=False):
         from .render import MultiRenderer, Renderer, default_context
         self.ctx = ctx or default_context()
         self.world, self.camera = world, camera
         self.spp, self.propagate_limit, self.absorptivity, self.seed = int(spp), int(propagate_limit), float(absorptivity), seed
         self.group, self.bands = group, int(bands)
         self.distributed = bool(distributed)
+        self.denoise = bool(denoise)
+        self.feature_passes = 0  # pt_render_features calls made (one per pose)
+        if self.denoise and self.distributed:
+            from .multigpu import _dist_active
+            if _dist_active(self.group):
+                raise ValueError("LegacyRenderer: denoise=True needs the sum of squares, which the process-group path does "
+                                 "not reduce; pass distributed=False, or devices= to split passes within this process")
         if devices is not None:
             from .multigpu import _dist_active
             if self.distributed and _dist_active(self.group):
                 raise ValueError("LegacyRenderer: devices= splits passes within this process; with an active process group "
                                  "pass distributed=False (or leave devices=None to split over the ranks)")
-            self.renderer = MultiRenderer(camera.resolution[0], camera.resolution[1], devices, self.ctx)
+            self.renderer = MultiRenderer(camera.resolution[0], camera.resolution[1], devices, self.ctx, want_sq=self.denoise)
         else:
-            self.renderer = Renderer(camera.resolution[0], camera.resolution[1], self.ctx)
+            self.renderer = Renderer(camera.resolution[0], camera.resolution[1], self.ctx, want_sq=self.denoise)
         self.frame = None
         self._total = 0       # samples per pixel in the image (over all ranks)
         self._partial = None  # ranks > 0: scratch accumulator of one pass
@@ -735,6 +745,9 @@ class LegacyRenderer:
             self._total = 0
         first = self._total if spp_offset is None else int(spp_offset)
         scene = self.world.device_scene(self.ctx)
+        if self.denoise and (moved or self.feature_passes == 0):
+            self.renderer.features(scene, self.camera.to_struct(), 4, self.seed, 0, 0, _lib.PT_SHADE_LEGACY)
+            self.feature_passes += 1
         if ws == 1:
             self.renderer.render(scene, self.camera.to_struct(), self.spp, self.propagate_limit, _lib.PT_SHADE_LEGACY,
                                  self.seed, spp_offset=first, absorptivity=self.absorptivity, want_stats=False)
@@ -755,7 +768,7 @@ class LegacyRenderer:
         if rank != 0:
             self.frame = None
             return None
-        self.frame = self.renderer.image(aces=False, gamma=2.2, total_spp=self._total)
+        self.frame = self.renderer.image(aces=False, gamma=2.2, total_spp=self._total, denoise=self.denoise)
         return self.frame
 
     def frames(self, camera_path, passes_per_pose=1):

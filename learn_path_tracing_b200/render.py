@@ -41,11 +41,17 @@ class Renderer:
         self.accum_sq = torch.zeros_like(self.accum) if want_sq else None
         self.spp_done = 0
         self.last_stats = None
+        self.feature_planes = None  # first-hit guide features (features()), allocated on first use
+        self.feature_spp = 0        # samples per pixel in feature_planes
+        self._denoised = None
 
     def clear(self):
         self.accum.zero_()
         if self.accum_sq is not None:
             self.accum_sq.zero_()
+        if self.feature_planes is not None:
+            self.feature_planes.zero_()
+        self.feature_spp = 0
         self.spp_done = 0
 
     def render(self, scene: _lib.Scene, cam: _lib.PtCamera, spp: int, max_depth: int,
@@ -88,6 +94,44 @@ class Renderer:
         p.reserved[1] = int(segments_per_launch)  # fused: ray segments per path slot per launch (0 = 32)
         return p
 
+    def features(self, scene: _lib.Scene, cam: _lib.PtCamera, spp: int = 4, seed: int = 1, spp_offset: int = 0,
+                 flags: int = 0, shading_model: int = _lib.PT_SHADE_V2):
+        """ADDS the first-hit guide features (normal, depth, albedo; pt_render_features) of samples
+        [spp_offset, spp_offset + spp) of the camera rays of render(..., seed, flags) into self.feature_planes, shaped
+        (2, H*W, 4), and returns it.  clear() zeroes it.  Computed on this renderer's own context (a MultiRenderer's
+        root): they cost a few camera rays, not paths."""
+        if self.feature_planes is None:
+            self.feature_planes = self.torch.zeros((2, self.height * self.width, 4), dtype=self.torch.float32,
+                                                   device=self.accum.device)
+        p = self._params(spp, 1, shading_model, seed, spp_offset, 0.25, 0, 0, 0, 0, 0, 0)
+        p.flags = int(flags)
+        self.ctx.set_stream(self.torch.cuda.current_stream(self.accum.device).cuda_stream)
+        self.ctx.render_features(scene, cam, p, self.feature_planes.data_ptr())
+        self.feature_spp += int(spp)
+        return self.feature_planes
+
+    def denoised(self, iterations: int = 5, sigma_l: float = 0.0, sigma_n: float = 0.0, sigma_z: float = 0.0,
+                 total_spp: int | None = None):
+        """The denoised mean radiance (pt_denoise) as a float4 device tensor (H*W, 4), w = 1: the accumulators divided by
+        total_spp (default: the samples rendered), filtered under the guidance of self.feature_planes.  Needs
+        want_sq=True and features(); sigma 0 = the library's defaults."""
+        if self.feature_planes is None:
+            raise _lib.PtError("denoised(): no guide features yet; call features(scene, cam, ...) first")
+        if self.accum_sq is None:
+            raise _lib.PtError("denoised(): the filter needs the sum of squares: create the renderer with want_sq=True")
+        if self._denoised is None:
+            self._denoised = self.torch.empty_like(self.accum)
+        n = total_spp if total_spp is not None else max(self.spp_done, 1)
+        # pt_denoise divides the albedo plane by the accumulator's spp: features of another sample count (4 spp under an
+        # 8192-spp render) are rescaled to it.  Depth (t sum / hit count) and the normal direction are ratios: unchanged.
+        f = self.feature_planes
+        if self.feature_spp not in (0, n):
+            f = f * (n / self.feature_spp)
+        self.ctx.set_stream(self.torch.cuda.current_stream(self.accum.device).cuda_stream)
+        self.ctx.denoise(self.accum.data_ptr(), self.accum_sq.data_ptr(), f.data_ptr(), self.width, self.height, n,
+                         self._denoised.data_ptr(), iterations, sigma_l, sigma_n, sigma_z)
+        return self._denoised
+
     def side_stream(self):
         """A second CUDA stream of this renderer (reduce of one row band beside the rendering of the next)."""
         if getattr(self, "_side", None) is None:
@@ -110,10 +154,20 @@ class Renderer:
         q = self.ctx.download_accum(self.accum_sq.data_ptr(), self.width, self.height)
         return s, q
 
-    def image(self, aces: bool = True, gamma: float = 2.2, total_spp: int | None = None) -> np.ndarray:
-        """post_processing (ACES + gamma, __main__.py:90-96) or legacy gamma_correction (aces=False)."""
+    def image(self, aces: bool = True, gamma: float = 2.2, total_spp: int | None = None, denoise: bool = False) -> np.ndarray:
+        """post_processing (ACES + gamma, __main__.py:90-96) or legacy gamma_correction (aces=False).  denoise=True
+        tonemaps the denoised mean (denoised(), default filter settings) instead of the raw one."""
         n = total_spp if total_spp is not None else max(self.spp_done, 1)
+        if denoise:
+            d = self.denoised(total_spp=n)
+            return self.ctx.postprocess_host(d.data_ptr(), self.width, self.height, 1.0, aces, gamma)
         return self.ctx.postprocess_host(self.accum.data_ptr(), self.width, self.height, 1.0 / n, aces, gamma)
+
+
+def denoised_mean(r: Renderer, total_spp: int | None = None) -> np.ndarray:
+    """The denoised linear radiance of a renderer, Taichi field layout [W,H,3] (as Renderer.mean())."""
+    d = r.denoised(total_spp=total_spp)
+    return r.ctx.download_accum(d.data_ptr(), r.width, r.height)
 
 
 def resolve_devices(devices, root_device: int) -> list[int]:
@@ -197,16 +251,23 @@ class MultiRenderer(Renderer):
 
 def render(world, camera, spp: int = 8192, propagate_limit: int = 32, seed: int = 1, bsdf=None,
            ctx: _lib.Context | None = None, return_stats: bool = False, postprocess: bool = True,
-           pixel_grid: bool = False, absorptivity: float = 0.25, aces: bool = True, devices=None):
+           pixel_grid: bool = False, absorptivity: float = 0.25, aces: bool = True, devices=None, denoise: bool = False):
     """Drop-in for the v2 scripts' render(world, camera) + post_processing(): returns the tonemapped
     image as a float32 [W,H,3] array in Taichi field layout (pass it to imwrite).
     devices: None renders on `ctx` alone; a list of CUDA device indices (or "all") splits the frame over them in this
-    process (MultiRenderer; the first device must be the context's)."""
+    process (MultiRenderer; the first device must be the context's).
+    denoise=True returns the denoised image instead (Renderer.denoised(): 4-spp guide features of the render's camera
+    rays, five filter passes)."""
     ctx = ctx or default_context()
     w, h = camera.resolution
     model = getattr(bsdf, "shading_model", _lib.PT_SHADE_V2)
-    r = Renderer(w, h, ctx) if devices is None else MultiRenderer(w, h, devices, ctx)
-    st = r.render(world.device_scene(ctx), camera.to_struct(), spp, propagate_limit, model, seed, absorptivity=absorptivity,
-                  flags=_lib.PT_FLAG_PIXEL_GRID if pixel_grid else 0)  # stages 2-4: lattice rays, no jitter
-    img = r.image(aces=aces, gamma=2.2) if postprocess else r.mean()  # stages <= 5 write the linear image
+    r = Renderer(w, h, ctx, want_sq=denoise) if devices is None else MultiRenderer(w, h, devices, ctx, want_sq=denoise)
+    flags = _lib.PT_FLAG_PIXEL_GRID if pixel_grid else 0  # stages 2-4: lattice rays, no jitter
+    scene, cam = world.device_scene(ctx), camera.to_struct()
+    st = r.render(scene, cam, spp, propagate_limit, model, seed, absorptivity=absorptivity, flags=flags)
+    if denoise:
+        r.features(scene, cam, 4, seed, 0, flags, model)
+        img = r.image(aces=aces, gamma=2.2, denoise=True) if postprocess else denoised_mean(r)
+    else:
+        img = r.image(aces=aces, gamma=2.2) if postprocess else r.mean()  # stages <= 5 write the linear image
     return (img, st) if return_stats else img
